@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- appearance-optimisation steps/s (BASELINE.json metric) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): one train_clip step = render 512 rays x (64+64) samples through the 8x256
 SDF + 4x256 colour MLPs (placement + fine pass), shading/canvas/losses on a 224x224 canvas, CLIP ViT-B/32 on the
@@ -215,6 +215,33 @@ def count_my_launches(fn):
         return None, None, {"error": repr(e)}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def step_outputs(tr, loss):
+    """What one training step hands its caller, copied to the host: the loss, the CLIP cosines and image embeddings, the
+    loss stage's scalars, every render output, the flat gradient and the flat parameters / Adam moments after the update."""
+    arrays = {"loss": loss, "clip_cos": tr.cos, "clip_image_embedding": tr.emb, "loss_scalars": tr.scalars,
+              "grad": tr.grad, "params": tr.fp.flat, "adam_exp_avg": tr.exp_avg, "adam_exp_avg_sq": tr.exp_avg_sq}
+    arrays.update({"render_" + k: v for k, v in tr._out.items() if torch.is_tensor(v)})
+    out = {}
+    for k, v in arrays.items():
+        v = v.detach().cpu()
+        out[k] = v.double().numpy() if v.dtype == torch.float64 or not v.is_floating_point() else v.float().numpy()
+    return out
+
+
+def write_outputs(directory, arrays):
+    """One DIR/<name>.npy per array (float32, or float64 where the value is not a float32 tensor)."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES} byte budget")
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), a)
+
+
 def run_native(args):
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -299,10 +326,12 @@ def run_native(args):
 
     ev[0].record()
     for i in range(K):
-        one_step(i)
+        loss = one_step(i)
     ev[1].record()
     barrier()
     ms_value = ev[0].elapsed_time(ev[1])
+    # the steps below (render-only timing, phases, end to end) train on: snapshot the timed path's last step now
+    dumped = step_outputs(tr, loss) if args.dump_outputs and rank == 0 else None
     clocks = sampler.stop() if rank == 0 else None
 
     # render-only share (events around the two render calls) for the roofline of the MLP contractions
@@ -448,6 +477,10 @@ def run_native(args):
             line["parity"] = parity
             if args.ref_gpu:
                 line["ref_gpu"] = reference_gpu(sp, cp, clip_sd, text, device, steps=max(5, min(K, 20)))
+        if dumped is not None:
+            write_outputs(args.dump_outputs, dumped)
+            line["dump_outputs"] = {"dir": args.dump_outputs, "arrays": sorted(dumped),
+                                    "step": "last timed step (after warm-up, the profiled step and the timed steps)"}
         real_stdout.emit(json.dumps(line))
     if world > 1:
         tr.release_graph()          # the graph may hold the NCCL all-reduce: it has to go before the communicator
@@ -777,7 +810,14 @@ def main():
                     help="skip the cpu_baseline / parity / ref_gpu legs (kernel experiments)")
     ap.add_argument("--cpu-budget-s", type=float, default=20.0, help="CPU seconds the cpu_baseline leg may spend on steps")
     ap.add_argument("--ref-gpu", type=int, default=1, help="1: also time the unmodified reference renderer on this GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (loss, CLIP cosines, render outputs, gradient, parameters "
+                         "after the update) as DIR/<name>.npy; the inputs are seeded, so two builds can be compared array by array")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "native" or args.config != 1):
+        ap.error("--dump-outputs is available for the native arm of configs[1]")
     if args.warmup < 3 and args.impl == "native":
         args.warmup = 3
     if args.impl == "reference":

@@ -1,10 +1,22 @@
 """HOCON-subset reader: accessor API of pyhocon's ConfigTree as the reference uses it (main.py:39-127)."""
 import glob
 import os
+import tarfile
 
 import pytest
 
 from avatarclip_b200 import conf
+
+SHIPPED = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "shipped_confs.tar.xz")
+
+
+@pytest.fixture(scope="module")
+def shipped_confs(tmp_path_factory):
+    """The reference's confs/ tree as it ships (180 files, stored verbatim in tests/golden by oracle/pin_host_mirrors.py)."""
+    d = tmp_path_factory.mktemp("shipped")
+    with tarfile.open(SHIPPED) as tf:
+        tf.extractall(d, filter="data")
+    return str(d)
 
 SAMPLE = """
 general {
@@ -46,9 +58,8 @@ def test_sample():
         c["dataset.template_obj"]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference checkout only exists in the build container")
-def test_all_shipped_confs_parse():
-    files = glob.glob("/root/reference/AvatarGen/AppearanceGen/confs/**/*.conf", recursive=True)
+def test_all_shipped_confs_parse(shipped_confs):
+    files = glob.glob(os.path.join(shipped_confs, "confs/**/*.conf"), recursive=True)
     assert len(files) == 180
     for f in files:
         c = conf.parse_file(f)
@@ -58,14 +69,13 @@ def test_all_shipped_confs_parse():
         assert c.get_float("train.learning_rate") > 0
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference checkout only exists in the build container")
-def test_every_shipped_conf_constructs_its_networks_and_is_a_supported_loop():
+def test_every_shipped_conf_constructs_its_networks_and_is_a_supported_loop(shipped_confs):
     """All 180 shipped confs: the model subtrees are accepted as constructor kwargs (main.py:137-151) -- 3 distinct network
     configurations, incl. the extra_color-less one of base_models/astrongman.conf -- and the train.* switches name a loop the
     Runner implements (train_clip: use_silhouettes + extra_color; --mode train: astrongman.conf)."""
     import json
     import avatarclip_b200 as ab
-    files = sorted(glob.glob("/root/reference/AvatarGen/AppearanceGen/confs/**/*.conf", recursive=True))
+    files = sorted(glob.glob(os.path.join(shipped_confs, "confs/**/*.conf"), recursive=True))
     built, n_clip = {}, 0
     for f in files:
         c = conf.parse_file(f)

@@ -12,6 +12,7 @@ from oracle import loss as ol
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CONF = os.path.join(HERE, "runner_conf_sample.conf")
+GOLDEN = os.path.join(HERE, "golden")
 
 
 def _conf_text(tmp_path, data_dir=None, edits=()):
@@ -297,16 +298,35 @@ def test_extract_geometry_sphere_is_watertight_and_outward(tmp_path):
     assert torch.equal(sdf.sdf_hidden_appearance(pts.cuda()).cpu(), out)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/AvatarGen/AppearanceGen"),
-                    reason="reference checkout only exists in the build container")
+def _shipped_checkpoint(path):
+    """pretrained_models/zero_beta_stand_pose.pth's three network state dicts, rebuilt from the tensors tests/golden/neus_shipped.pt
+    carries, in the file's key order, each tensor checked against the sha256 recorded from the shipped file
+    (oracle/pin_host_mirrors.py)."""
+    import hashlib
+    g = torch.load(os.path.join(GOLDEN, "neus_shipped.pt"), weights_only=False)
+    ref = json.load(open(os.path.join(GOLDEN, "host_mirrors.json")))["checkpoint"]
+    src = {"sdf_network_fine": g["sdf_state"], "color_network_fine": g["col_state"], "variance_network_fine": {"variance": g["variance"]}}
+    ck = {}
+    for part, want in ref.items():
+        ck[part] = {k: src[part][k].clone() for k in want["keys"]}
+        for (k, v), h in zip(ck[part].items(), want["sha256"]):
+            assert hashlib.sha256(np.ascontiguousarray(v.numpy()).tobytes()).hexdigest() == h, (part, k)
+    torch.save(ck, path)
+    return ck
+
+
 def test_shipped_example_conf_constructs_a_runner_and_loads_the_shipped_checkpoint(tmp_path):
-    """confs/examples/ironman.conf as shipped (only the three relative paths made absolute, because the reference tree is
-    read-only and the test does not run from inside it): the Runner builds the networks from the conf subtrees, reads every
-    train.* key and loads `train.pretrain` = pretrained_models/zero_beta_stand_pose.pth like main.py:153-160,612-619."""
+    """confs/examples/ironman.conf as shipped (only the three relative paths made absolute, because the test does not run from
+    inside the reference tree): the Runner builds the networks from the conf subtrees, reads every train.* key and loads
+    `train.pretrain` = pretrained_models/zero_beta_stand_pose.pth like main.py:153-160,612-619."""
+    import tarfile
     from avatarclip_b200.runner import Runner
-    ag = "/root/reference/AvatarGen/AppearanceGen"
-    text = open(os.path.join(ag, "confs/examples/ironman.conf")).read()
-    for old, new in (("./exp/", str(tmp_path / "exp") + "/"), ("./data/", ag + "/data/"), ("./pretrained_models/", ag + "/pretrained_models/")):
+    with tarfile.open(os.path.join(GOLDEN, "shipped_confs.tar.xz")) as tf:
+        text = tf.extractfile("confs/examples/ironman.conf").read().decode()
+    (tmp_path / "pretrained_models").mkdir()
+    ck = _shipped_checkpoint(str(tmp_path / "pretrained_models" / "zero_beta_stand_pose.pth"))
+    for old, new in (("./exp/", str(tmp_path / "exp") + "/"), ("./data/", str(tmp_path / "data") + "/"),
+                     ("./pretrained_models/", str(tmp_path / "pretrained_models") + "/")):
         assert old in text
         text = text.replace(old, new)
     p = tmp_path / "ironman.conf"
@@ -314,7 +334,6 @@ def test_shipped_example_conf_constructs_a_runner_and_loads_the_shipped_checkpoi
     r = Runner(str(p), mode="validate", case="smpl", device="cpu")
     assert (r.use_silhouettes, r.add_no_texture, r.texture_cast_light, r.use_face_prompt, r.use_back_prompt, r.extra_color) == (True,) * 6
     assert r.max_ray_num == 112 * 112 and r.end_iter == 100000 and r.renderer.n_samples == 32 and r.renderer.n_importance == 32
-    ck = torch.load(os.path.join(ag, "pretrained_models/zero_beta_stand_pose.pth"), map_location="cpu", weights_only=False)
     for k, v in ck["sdf_network_fine"].items():
         assert torch.equal(r.sdf_network.state_dict()[k], v), k
     assert torch.equal(r.deviation_network.variance.detach(), ck["variance_network_fine"]["variance"])

@@ -1,20 +1,30 @@
-"""Runner.train (--mode train, the NeuS pre-fit) against the reference's own loop text (main.py:180-256 + :568-586) executed in
-place on the CPU: same fake dataset (random pixel batches from torch's global generator), same differentiable fake renderer
-over the network parameters, `torch.optim.Adam`, identical seeds.  Pins the loop's host logic -- image permutation cycling,
-mask handling, the loss formula, optimiser stepping, WHEN the learning rate is updated, what is logged under which name -- not
-the renderer (GPU parity tests).  Build container only."""
-import copy
+"""Runner.train (--mode train, the NeuS pre-fit) against the reference's own loop text (main.py:180-256 + :568-586) on the CPU:
+same fake dataset (random pixel batches from torch's global generator), same differentiable fake renderer over the network
+parameters, `torch.optim.Adam`, identical seeds.  Pins the loop's host logic -- image permutation cycling, mask handling, the
+loss formula, optimiser stepping, WHEN the learning rate is updated, what is logged under which name -- not the renderer (GPU
+parity tests).  The reference side was recorded by executing those lines in place on the same fakes
+(oracle/pin_host_mirrors.py -> tests/golden/host_mirrors.{json,npz})."""
+import json
 import os
-import textwrap
-import types
 
+import numpy as np
 import pytest
 import torch
-import torch.nn.functional as F
 
-REF_MAIN = "/root/reference/AvatarGen/AppearanceGen/main.py"
 HERE = os.path.dirname(os.path.abspath(__file__))
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_MAIN), reason="reference checkout only exists in the build container")
+GOLDEN = os.path.join(HERE, "golden")
+CLIP_STEPS = 48
+CLIP_CONF_EDITS = (("warm_up_end = 500", "warm_up_end = 5"), ("end_iter = 100000", "end_iter = 80"))
+
+
+def TRAIN_CONF_EDITS(mask_weight, white):
+    return (("end_iter = 100000", "end_iter = 12"), ("warm_up_end = 500", "warm_up_end = 4"), ("batch_size = 512", "batch_size = 40"),
+            ("mask_weight = 0.5", f"mask_weight = {mask_weight}"), ("use_white_bkgd = False", f"use_white_bkgd = {white}"),
+            ("report_freq = 100", "report_freq = 3"))
+
+
+def _golden():
+    return json.load(open(os.path.join(GOLDEN, "host_mirrors.json")))
 
 
 class FakeDataset:
@@ -55,81 +65,57 @@ class Writer:
         self.rec.append((name, float(value), int(step)))
 
 
-def _reference_methods():
-    lines = open(REF_MAIN).read().split("\n")
-    assert lines[179].strip() == "def train(self):" and "image_perm = self.get_image_perm()" in lines[255]
-    assert lines[567].strip() == "def get_image_perm(self):" and "g['lr']" in lines[585]
-    ns = dict(np=__import__("numpy"), torch=torch, F=F, os=os, tqdm=lambda it: it)
-    exec(textwrap.dedent("\n".join(lines[179:256])), ns)
-    exec(textwrap.dedent("\n".join(lines[567:586])), ns)
-    return ns
-
-
 @pytest.mark.parametrize("mask_weight,white", [(0.5, False), (0.0, True)])
-def test_mode_train_loop_equals_the_reference_loop(tmp_path, mask_weight, white, capsys):
+def test_mode_train_loop_equals_the_reference_loop(tmp_path, mask_weight, white):
     from avatarclip_b200.runner import Runner
     conf = open(os.path.join(HERE, "runner_conf_sample.conf")).read().replace("./exp/CASE_NAME/demo", str(tmp_path / "ours"))
-    for old, new in (("end_iter = 100000", "end_iter = 12"), ("warm_up_end = 500", "warm_up_end = 4"), ("batch_size = 512", "batch_size = 40"),
-                     ("mask_weight = 0.5", f"mask_weight = {mask_weight}"), ("use_white_bkgd = False", f"use_white_bkgd = {white}"),
-                     ("report_freq = 100", "report_freq = 3")):
+    for old, new in TRAIN_CONF_EDITS(mask_weight, white):
         assert old in conf
         conf = conf.replace(old, new)
     p = tmp_path / "c.conf"
     p.write_text(conf)
     r = Runner(str(p), mode="train", case="smpl", device="cpu")
     r.dataset = FakeDataset()
-    # the reference side: independent copies of the same networks, torch.optim.Adam over sdf + variance + colour (main.py:141-145)
-    nets = [copy.deepcopy(m) for m in (r.sdf_network, r.deviation_network, r.color_network)]
-    ref_params = [q for m in nets for q in m.parameters()]
-    ns = _reference_methods()
-    wr_ref = Writer()
-    ns["SummaryWriter"] = lambda log_dir=None: wr_ref
-    ref = types.SimpleNamespace(
-        base_exp_dir=str(tmp_path / "ref"), end_iter=12, iter_step=0, dataset=FakeDataset(), batch_size=40, use_white_bkgd=white,
-        mask_weight=mask_weight, igr_weight=r.igr_weight, report_freq=3, save_freq=10 ** 9, val_freq=10 ** 9, val_mesh_freq=10 ** 9,
-        warm_up_end=4.0, anneal_end=0.0, learning_rate=r.learning_rate, learning_rate_alpha=r.learning_rate_alpha,
-        renderer=types.SimpleNamespace(render=make_render(ref_params)), optimizer=torch.optim.Adam(ref_params, lr=r.learning_rate))
-    for name in ("get_image_perm", "get_cos_anneal_ratio", "update_learning_rate"):
-        setattr(ref, name, types.MethodType(ns[name], ref))
-    torch.manual_seed(7)
-    ns["train"](ref)
-    ref_out = capsys.readouterr().out
-    # our side
+    key = f"{mask_weight}_{white}"
+    ref = _golden()["train_loop"][key]
+    arrays = np.load(os.path.join(GOLDEN, "host_mirrors.npz"))
     wr = Writer()
     r._make_writer = lambda: wr
     r.save_freq = r.val_freq = r.val_mesh_freq = 10 ** 9
     r.renderer.render = make_render(r._all_params())
     torch.manual_seed(7)
     logs = []
-    assert r.train(log=logs.append, validate=False) == 12 == ref.iter_step
-    assert [n for n, _, _ in wr.rec] == [n for n, _, _ in wr_ref.rec]                # same scalar names in the same order
-    assert [s for _, _, s in wr.rec] == [s for _, _, s in wr_ref.rec]
-    worst = max(abs(a - b) / max(abs(b), 1e-12) for (_, a, _), (_, b, _) in zip(wr.rec, wr_ref.rec))
+    assert r.train(log=logs.append, validate=False) == 12 == ref["iter_step"]
+    assert [n for n, _, _ in wr.rec] == [n for n, _, _ in ref["rec"]]                # same scalar names in the same order
+    assert [s for _, _, s in wr.rec] == [s for _, _, s in ref["rec"]]
+    worst = max(abs(a - b) / max(abs(b), 1e-12) for (_, a, _), (_, b, _) in zip(wr.rec, ref["rec"]))
     assert worst < 1e-6, worst
-    for a, b in zip(r._all_params(), ref_params):                                    # the same parameters after 12 Adam steps
-        assert torch.allclose(a.detach(), b.detach(), rtol=1e-6, atol=1e-9)
-    assert r.optimizer.param_groups[0]["lr"] == ref.optimizer.param_groups[0]["lr"]
+    params = list(r._all_params())                                                   # the same parameters after 12 Adam steps
+    assert len(params) == ref["n_params"] and [list(q.shape) for q in params] == ref["param_shapes"]
+    for i, a in enumerate(params):                                                   # on a fixed, seeded sample of each tensor
+        idx = torch.from_numpy(arrays[f"train_loop_{key}_param{i}_idx"]).long()
+        want = torch.from_numpy(arrays[f"train_loop_{key}_param{i}_val"])
+        assert torch.allclose(a.detach().reshape(-1)[idx], want, rtol=1e-6, atol=1e-9), i
+    assert r.optimizer.param_groups[0]["lr"] == ref["final_lr"]
     lr_ours = [str(m).split("lr=")[1] for m in logs if "lr=" in str(m)]
-    lr_ref = [l.split("lr=")[1] for l in ref_out.splitlines() if "lr=" in l]
-    assert lr_ours == lr_ref and len(lr_ours) == 4                                   # the lr in force at steps 3, 6, 9, 12
+    assert lr_ours == ref["lr_printed"] and len(lr_ours) == 4                        # the lr in force at steps 3, 6, 9, 12
 
 
 def test_train_clip_host_logic_equals_the_reference_lines(tmp_path, monkeypatch):
     """What Runner.train_clip hands to the fused step, step by step -- camera pose, background mode, light, ambience (numpy's
     global stream seeded by train.seed), WHICH cached text embedding (main.py:499-507: face every 4th step, back when the camera
     is behind, else body), the learning rate in force (update_learning_rate before the loop and after every step, :339,563)
-    and the cosine-anneal ratio -- against the reference's own lines executed in place.  The step itself is mocked (GPU tests)."""
-    import numpy as np
+    and the cosine-anneal ratio -- against what the reference's own lines gave for the same seed and conf.  The step itself is
+    mocked (GPU tests)."""
+    import types
     from avatarclip_b200 import views
     from avatarclip_b200.runner import Runner
-    from oracle.pin_loss_stage import cut
-    from oracle.pin_sampling import reference_draws
     conf = open(os.path.join(HERE, "runner_conf_sample.conf")).read().replace("./exp/CASE_NAME/demo", str(tmp_path / "ours"))
-    conf = conf.replace("warm_up_end = 500", "warm_up_end = 5").replace("end_iter = 100000", "end_iter = 80")
+    for old, new in CLIP_CONF_EDITS:
+        conf = conf.replace(old, new)
     p = tmp_path / "c.conf"
     p.write_text(conf)
     r = Runner(str(p), mode="train_clip", case="smpl", device="cpu")                  # seeds numpy with train.seed = 11
-    n_steps = 48
     body, face, back = torch.zeros(1, 4), torch.ones(1, 4), torch.full((1, 4), 2.0)
     r.encoded_text, r.encoded_face_text, r.encoded_back_text = body, face, back
     r.clip_tower, r.v, r.f = object(), torch.zeros(1, 3, 3), np.zeros((1, 3), dtype=np.int64)
@@ -161,25 +147,13 @@ def test_train_clip_host_logic_equals_the_reference_lines(tmp_path, monkeypatch)
     r.trainer = FakeTrainer()
     monkeypatch.setattr(views, "ViewBuilder", FakeBuilder)
     r._make_writer = lambda: __import__("avatarclip_b200.runner", fromlist=["_NullWriter"])._NullWriter()
-    assert r.train_clip(max_steps=n_steps, log=lambda m: None, validate=False) == n_steps
-    # ---- the reference's lines
-    ref = reference_draws(r.seed, n_steps + 1, r.head_height, face=True, bg_aug=True, shading=True)   # ours looks one step ahead
-    prompt_lines = cut("main.py", 499, 507, "if self.use_face_prompt and iter_i % 4 == 0", "current_no_texture_text_encoding = self.encoded_text")
-    sched = {"np": np}
-    exec(cut("main.py", 571, 586, "def get_cos_anneal_ratio", "g['lr']"), sched)
-    for i, got in enumerate(rec):
-        s = types.SimpleNamespace(use_face_prompt=True, use_back_prompt=True, encoded_text=body, encoded_face_text=face,
-                                  encoded_back_text=back)
-        loc = dict(self=s, iter_i=i, is_front=ref[i]["is_front"])
-        exec(prompt_lines, loc)
-        assert got["text"] == float(loc["current_text_encoding"][0, 0]), i
-        assert float(loc["current_no_texture_text_encoding"][0, 0]) == got["text"]
-        sch = types.SimpleNamespace(iter_step=i, warm_up_end=5.0, end_iter=80, learning_rate_alpha=r.learning_rate_alpha,
-                                    learning_rate=r.learning_rate, anneal_end=0.0,
-                                    optimizer=types.SimpleNamespace(param_groups=[{"lr": None}]))
-        sched["update_learning_rate"](sch)
-        assert got["lr"] == sch.optimizer.param_groups[0]["lr"], i
-        assert got["cos_anneal"] == float(sched["get_cos_anneal_ratio"](sch))
-        assert np.array_equal(got["pose"], np.asarray(ref[i]["pose"])) and got["bg"] == ref[i]["choice_i"], i
-        assert np.array_equal(got["light"], np.asarray(ref[i]["light_dir"]).astype(np.float32)) and got["ambience"] == ref[i]["ambience"]
+    assert r.train_clip(max_steps=CLIP_STEPS, log=lambda m: None, validate=False) == CLIP_STEPS
+    ref = _golden()["train_clip"]
+    assert len(ref) == len(rec) == CLIP_STEPS
+    for i, (got, want) in enumerate(zip(rec, ref)):
+        assert got["text"] == want["text"] == want["no_texture_text"], i
+        assert got["lr"] == want["lr"], i
+        assert got["cos_anneal"] == want["cos_anneal"]
+        assert np.array_equal(got["pose"], np.asarray(want["pose"])) and got["bg"] == want["bg"], i
+        assert np.array_equal(got["light"], np.asarray(want["light"], dtype=np.float32)) and got["ambience"] == want["ambience"]
     assert {g["text"] for g in rec} == {0.0, 1.0, 2.0}             # body, face and back prompts all occurred

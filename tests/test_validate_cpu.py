@@ -1,17 +1,20 @@
 """Runner.validate_image's host side (batching, normal-image rotation, scaling, file names, image layout) against the reference's
-own method text (main.py:741-820) executed in place, both driven by the SAME fake dataset and the SAME fake renderer (deterministic
-functions of the rays, CPU tensors) -- the render itself is covered by the GPU parity tests.  Build container only."""
+own method text (main.py:741-820), both driven by the SAME fake dataset and the SAME fake renderer (deterministic functions of
+the rays, CPU tensors) -- the render itself is covered by the GPU parity tests.  The reference side was recorded by executing
+the methods in place on these fakes (oracle/pin_host_mirrors.py -> tests/golden/host_mirrors.{json,npz})."""
+import json
 import os
-import textwrap
-import types
 
 import numpy as np
 import pytest
 import torch
 
-REF_MAIN = "/root/reference/AvatarGen/AppearanceGen/main.py"
 HERE = os.path.dirname(os.path.abspath(__file__))
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_MAIN), reason="reference checkout only exists in the build container")
+GOLDEN = os.path.join(HERE, "golden")
+
+
+def _golden():
+    return json.load(open(os.path.join(GOLDEN, "host_mirrors.json"))), np.load(os.path.join(GOLDEN, "host_mirrors.npz"))
 
 
 class FakeDataset:
@@ -54,15 +57,6 @@ class FakeRenderer:
                 "weight_sum": w.sum(1, keepdim=True), "mid_z_vals": w}
 
 
-def _reference_validate_image():
-    import cv2 as cv
-    lines = open(REF_MAIN).read().split("\n")[740:820]
-    assert lines[0].strip().startswith("def validate_image(self, idx=-1, resolution_level=-1)") and "normal_img[..., i])" in lines[-1]
-    ns = dict(np=np, torch=torch, os=os, cv=cv)
-    exec(textwrap.dedent("\n".join(lines)), ns)
-    return ns["validate_image"]
-
-
 @pytest.mark.parametrize("extra_color", [True, False])
 def test_validate_image_files_equal_the_reference_methods(tmp_path, extra_color):
     import cv2 as cv
@@ -77,34 +71,17 @@ def test_validate_image_files_equal_the_reference_methods(tmp_path, extra_color)
     r.renderer.render = FakeRenderer().render
     r.renderer.n_samples, r.renderer.n_importance = 3, 2
     img, extra, normal = r.validate_image(idx=3, resolution_level=2)
-    ref_self = types.SimpleNamespace(dataset=FakeDataset(), iter_step=1234, batch_size=100, validate_resolution_level=1,
-                                     use_white_bkgd=False, extra_color=extra_color, renderer=FakeRenderer(),
-                                     base_exp_dir=str(tmp_path / "ref"), get_cos_anneal_ratio=lambda: 1.0)
-    _reference_validate_image()(ref_self, idx=3, resolution_level=2)
+    meta, arrays = _golden()
+    ref_files = meta["validate_image"][str(int(extra_color))]
     name = "00001234_0_3.png"
+    assert {d: sorted(os.listdir(os.path.join(str(tmp_path / "ours"), d))) for d in ref_files} == ref_files
     for d in ("validations_fine", "normals") + (("validations_extra_fine",) if extra_color else ()):
         a = cv.imread(os.path.join(str(tmp_path / "ours"), d, name), cv.IMREAD_UNCHANGED)
-        b = cv.imread(os.path.join(str(tmp_path / "ref"), d, name), cv.IMREAD_UNCHANGED)
-        assert a is not None and b is not None and a.shape == b.shape and np.array_equal(a, b), d
+        b = arrays[f"validate_image_{int(extra_color)}/{d}/{name}"]
+        assert a is not None and a.shape == b.shape and np.array_equal(a, b), d
     assert img.shape == (12, 12, 3) and normal.shape == (12, 12, 3) and (extra is None) == (not extra_color)
     if not extra_color:                       # the reference creates the directory but writes nothing into it
         assert os.listdir(os.path.join(str(tmp_path / "ours"), "validations_extra_fine")) == []
-
-
-def _reference_validate_mesh(captured):
-    lines = open(REF_MAIN).read().split("\n")[849:919]
-    assert lines[0].strip().startswith("def validate_mesh(self, world_space=False") and "logging.info('End')" in lines[-1]
-    import logging
-
-    class Trimesh:                      # stand-in for the absent trimesh package: records what would be exported
-        def __init__(self, vertices, triangles, vertex_colors=None):
-            captured.update(vertices=np.asarray(vertices), triangles=np.asarray(triangles), colors=np.asarray(vertex_colors))
-
-    tm = types.SimpleNamespace(Trimesh=Trimesh, exchange=types.SimpleNamespace(export=types.SimpleNamespace(
-        export_mesh=lambda mesh, path, file_type=None: captured.update(path=path, file_type=file_type))))
-    ns = dict(np=np, torch=torch, os=os, logging=logging, trimesh=tm, to8b=lambda x: (255 * np.clip(x, 0, 1)).astype(np.uint8))
-    exec(textwrap.dedent("\n".join(lines)), ns)
-    return ns["validate_mesh"]
 
 
 class MeshRenderer(FakeRenderer):
@@ -138,17 +115,9 @@ def test_validate_mesh_colours_equal_the_reference_methods(tmp_path, extra_color
     mr = MeshRenderer()
     r.renderer.render, r.renderer.extract_geometry = mr.render, mr.extract_geometry
     path = r.validate_mesh(resolution=64)
-    captured = {}
-    ds = FakeDataset()
-    ds.object_bbox_min, ds.object_bbox_max = np.array([-1.01] * 3), np.array([1.01] * 3)
-    ref_self = types.SimpleNamespace(dataset=ds, iter_step=77, batch_size=100, use_white_bkgd=False, extra_color=extra_color,
-                                     renderer=MeshRenderer(), base_exp_dir=str(tmp_path / "ref"), get_cos_anneal_ratio=lambda: 1.0)
-    saved_cuda = torch.Tensor.cuda
-    torch.Tensor.cuda = lambda self_, *a, **k: self_          # `.cuda()` (main.py:859,872): a device move, identity on this box
-    try:
-        _reference_validate_mesh(captured)(ref_self, resolution=64)
-    finally:
-        torch.Tensor.cuda = saved_cuda
+    meta, arrays = _golden()
+    captured = dict(meta["validate_mesh"][str(int(extra_color))],
+                    **{k: arrays[f"validate_mesh_{int(extra_color)}_{k}"] for k in ("vertices", "triangles", "colors")})
     v, f, c = read_ply(path)
     assert os.path.basename(path) == os.path.basename(captured["path"]) == "00000077.ply" and captured["file_type"] == "ply"
     assert np.array_equal(f, captured["triangles"].astype(np.int32)) and np.allclose(v, captured["vertices"].astype(np.float32))
@@ -156,57 +125,36 @@ def test_validate_mesh_colours_equal_the_reference_methods(tmp_path, extra_color
     assert np.array_equal(c, captured["colors"])                 # the same view wins for every vertex, the same 8-bit colour
 
 
+class CastLightDataset(FakeDataset):
+    def gen_rays_pose(self, pose, resolution_level=1):
+        pose = torch.as_tensor(np.asarray(pose), dtype=torch.float32)
+        n = int(self.H // resolution_level)
+        yy, xx = torch.meshgrid(torch.linspace(-1, 1, n), torch.linspace(-1, 1, n), indexing="ij")
+        d = torch.stack([xx, -yy, -torch.ones_like(xx)], -1)
+        d = d / d.norm(dim=-1, keepdim=True)
+        d = torch.sum(d[..., None, :] * pose[:3, :3], -1)
+        return pose[None, None, :3, 3].expand(d.shape), d
+
+
 def test_render_geometry_cast_light_equals_the_reference_method(tmp_path):
-    """main.py:634-739 executed in place (head close-up, one light draw, Lambert shading of the extra colour, ambience 0)
-    against Runner.render_geometry_cast_light under the same numpy seed, fake dataset and fake renderer."""
+    """main.py:634-739 (head close-up, one light draw, Lambert shading of the extra colour, ambience 0) against
+    Runner.render_geometry_cast_light under the same numpy seed, fake dataset and fake renderer."""
     import cv2 as cv
-    from torchvision import transforms
     from avatarclip_b200.runner import Runner
-    lines = open(REF_MAIN).read().split("\n")
-    body = lines[633:739]
-    assert body[0].strip().startswith("def render_geometry_cast_light(self)") and body[-1].strip() == ")"
-    uns = dict(np=np, torch=torch)
-    utils = open(os.path.join(os.path.dirname(REF_MAIN), "models", "utils.py")).read().split("\n")
-    exec(textwrap.dedent("\n".join(utils[5:27])), uns)            # norm_np_arr, lookat (models/utils.py:6-27)
-    exec(textwrap.dedent("\n".join(utils[58:64])), uns)          # sphere_coord (:59-64)
-    captured = {}
-    ns = dict(np=np, torch=torch, os=os, transforms=transforms, lookat=uns["lookat"], sphere_coord=uns["sphere_coord"],
-              imageio=types.SimpleNamespace(imwrite=lambda path, arr: captured.update(path=path, img=np.asarray(arr))),
-              to8b=lambda x: (255 * np.clip(x, 0, 1)).astype(np.uint8))
-    exec(textwrap.dedent("\n".join(body)), ns)
-
-    class DS(FakeDataset):
-        def gen_rays_pose(self, pose, resolution_level=1):
-            pose = torch.as_tensor(np.asarray(pose), dtype=torch.float32)
-            n = int(self.H // resolution_level)
-            yy, xx = torch.meshgrid(torch.linspace(-1, 1, n), torch.linspace(-1, 1, n), indexing="ij")
-            d = torch.stack([xx, -yy, -torch.ones_like(xx)], -1)
-            d = d / d.norm(dim=-1, keepdim=True)
-            d = torch.sum(d[..., None, :] * pose[:3, :3], -1)
-            return pose[None, None, :3, 3].expand(d.shape), d
-
     conf = open(os.path.join(HERE, "runner_conf_sample.conf")).read().replace("./exp/CASE_NAME/demo", str(tmp_path / "ours"))
     p = tmp_path / "c.conf"
     p.write_text(conf)
     r = Runner(str(p), mode="validate", case="smpl", device="cpu")
-    r.dataset, r.batch_size = DS(), 500
+    assert r.head_height == 0.55                                  # the value the reference side was run with
+    r.dataset, r.batch_size = CastLightDataset(), 500
     r.renderer.render = FakeRenderer().render
     r.renderer.n_samples, r.renderer.n_importance = 3, 2
     np.random.seed(21)
     path = r.render_geometry_cast_light()
     next_ours = np.random.uniform()
-    ref_self = types.SimpleNamespace(dataset=DS(), batch_size=500, head_height=r.head_height, renderer=FakeRenderer(),
-                                     base_exp_dir=str(tmp_path / "ref"), get_cos_anneal_ratio=lambda: 1.0)
-    os.makedirs(ref_self.base_exp_dir, exist_ok=True)
-    saved_cuda = torch.Tensor.cuda
-    torch.Tensor.cuda = lambda self_, *a, **k: self_
-    np.random.seed(21)
-    try:
-        ns["render_geometry_cast_light"](ref_self)
-        next_ref = np.random.uniform()
-    finally:
-        torch.Tensor.cuda = saved_cuda
+    meta, arrays = _golden()
+    ref, ref_img = meta["cast_light"], arrays["cast_light_img"]
     ours = cv.cvtColor(cv.imread(path, cv.IMREAD_UNCHANGED), cv.COLOR_BGR2RGB)
-    assert os.path.basename(path) == os.path.basename(captured["path"]) == "cast_light_texture_head_black.png"
-    assert ours.shape == captured["img"].shape == (48, 48, 3) and np.array_equal(ours, captured["img"])
-    assert next_ours == next_ref              # both sides consumed the same draws of numpy's global stream (main.py:671-674)
+    assert os.path.basename(path) == ref["path"] == "cast_light_texture_head_black.png"
+    assert ours.shape == ref_img.shape == (48, 48, 3) and np.array_equal(ours, ref_img)
+    assert next_ours == ref["next_uniform"]    # both sides consumed the same draws of numpy's global stream (main.py:671-674)
