@@ -18,7 +18,8 @@
 // HBM traffic per point: 160 B in (the encoded pair) + 4 B out, against 2 x 1 KB per layer and direction for the
 // unfused launches (8 launches per pass); L2 -> SM: 256 KB of weights per layer and 128-point tile.
 // Synchronisation: wfull/wempty (W ring), a0full (TMA tile input), afull (epilogue -> MMA: next A complete AND
-// accumulator drained, one arrival per epilogue warp), accfull (tcgen05.commit: accumulator complete, A reads done).
+// accumulator drained, one arrival per epilogue warp), accfull (tcgen05.commit: accumulator complete, A reads done),
+// afree (tcgen05.commit with the last layer's final slab, once per tile: the A tile may take the next tile's input).
 #include <cuda.h>
 
 #include <cstdlib>
@@ -88,7 +89,7 @@ k_sdf_chain(const __grid_constant__ Maps maps, const __grid_constant__ DevArgs a
   float* sdf_acc = (float*)(smem + kABytes + kWStages * kWSlab + kBarBytes);
   uint32_t* tmem_slot = (uint32_t*)(sdf_acc + kCM);
   const uint32_t wfull0 = smem_u32(bars), wempty0 = wfull0 + 8 * kWStages, a0full = wempty0 + 8 * kWStages,
-                 afull = a0full + 8, accfull = afull + 8;
+                 afull = a0full + 8, accfull = afull + 8, afree = accfull + 8;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int L = a.L;
 
@@ -98,6 +99,7 @@ k_sdf_chain(const __grid_constant__ Maps maps, const __grid_constant__ DevArgs a
     mbar_init(a0full, 1);
     mbar_init(afull, kEW);
     mbar_init(accfull, 1);
+    mbar_init(afree, 1);
     fence_barrier_init();
   }
   if (warp == 1) tmem_alloc(smem_u32(tmem_slot), kTmemCols);
@@ -114,8 +116,13 @@ k_sdf_chain(const __grid_constant__ Maps maps, const __grid_constant__ DevArgs a
       pdl_wait();            // the encoded points are the predecessor kernel's output (launched with launch_pdl: this
       pdl_trigger();         // CTA's set-up ran while that kernel was still draining)
       for (int tile = blockIdx.x; tile < a.tiles; tile += gridDim.x, ++lt) {
-        // the A buffer is free for the next tile's input once the last layer's MMAs of the previous tile completed
-        if (lt > 0) mbar_wait(accfull, (uint32_t)((lt * L - 1) & 1));
+        // the A buffer is free for the next tile's input once the last layer's MMAs of the previous tile completed.
+        // afree completes once per tile and its next phase needs this tile's input, so the producer is never more than
+        // one phase behind and the parity wait cannot be satisfied by an older phase.  (Waiting on accfull, which
+        // completes once per LAYER, could be: with a last layer of one k-block the 3-stage weight ring lets the producer
+        // get here before layer L-2 has committed, and the TMA load would overwrite the A tile that layer's epilogue
+        // is still writing.)
+        if (lt > 0) mbar_wait(afree, (uint32_t)((lt - 1) & 1));
         mbar_expect_tx(a0full, 2 * kASlab);
         tma_load_2d(sA, &maps.a0hi, 0, tile * kCM, a0full);
         tma_load_2d(sA + kASlab, &maps.a0lo, 0, tile * kCM, a0full);
@@ -130,6 +137,7 @@ k_sdf_chain(const __grid_constant__ Maps maps, const __grid_constant__ DevArgs a
             }
         }
       }
+      if (lt > 0) mbar_wait(afree, (uint32_t)((lt - 1) & 1));   // the last tile's arrival lands before the CTA exits
     }
     __syncwarp();
   } else if (warp == 1) {
@@ -168,7 +176,10 @@ k_sdf_chain(const __grid_constant__ Maps maps, const __grid_constant__ DevArgs a
                 }
               }
               umma_commit(wempty0 + 8 * s);
-              if (kb == nkb - 1 && h == 1) umma_commit(accfull);
+              if (kb == nkb - 1 && h == 1) {
+                umma_commit(accfull);
+                if (l == L - 1) umma_commit(afree);
+              }
             }
             __syncwarp();
           }

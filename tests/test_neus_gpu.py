@@ -106,22 +106,75 @@ def test_sdf_query_matches_oracle():
     assert U.rel_to_max(got, want) < 1e-5
 
 
-@pytest.mark.parametrize("name,P", [("tiny", 77), ("tiny", 5000), ("skiplast", 1000), ("shipped", 4099), ("b2", 20000)])
+# five full waves of 128-point tiles on 148 SMs plus a ragged tile: the busiest chain CTA walks 6 tiles
+P_PERSISTENT = 5 * 148 * 128 + 77
+
+
+def _chain_net(name, seed):
+    """(sdf_kw, col_kw, ren_kw, sdf_state, col_state, variance): a synthetic case or the weights of a golden vector."""
+    if name in U.CASES:
+        sdf_kw, col_kw, ren_kw, _ = U.CASES[name]
+        sp, cp = U.synth_state(sdf_kw, col_kw, seed)
+        return sdf_kw, col_kw, ren_kw, sp, cp, 0.3
+    b = torch.load(os.path.join(U.GOLDEN, f"neus_{name}.pt"), map_location="cpu", weights_only=False)
+    return b["sdf_kw"], b["col_kw"], b["ren_kw"], b["sdf_state"], b["col_state"], b["variance"]
+
+
+def _chain_query_errors(name, P, chunk=4096):
+    """sdf_query of engine 1 on P points against the fp64 oracle, with the fused chain (default) and with the
+    layer-by-layer launches (AVC_FUSED_CHAIN=0).  Returns {variant: rel-to-max error}."""
+    sdf_kw, col_kw, ren_kw, sp, cp, variance = _chain_net(name, 5)
+    sconf, cconf, rconf = U.confs_from_kw(sdf_kw, col_kw, ren_kw)
+    sdf, col, var, ren = U.build_product(sdf_kw, col_kw, ren_kw, sp, cp, variance, "cuda", engine=1, chunk=chunk)
+    pts = (torch.rand(P, 3, generator=torch.Generator().manual_seed(P)) - 0.5) * 2
+    from oracle import neus
+    want = neus.sdf_value({k: v.double() for k, v in sp.items()}, sconf, pts.double())
+    errs = {}
+    saved = os.environ.get("AVC_FUSED_CHAIN")
+    try:
+        for variant, env in (("fused", None), ("layered", "0")):
+            if env is None:
+                os.environ.pop("AVC_FUSED_CHAIN", None)
+            else:
+                os.environ["AVC_FUSED_CHAIN"] = env
+            errs[variant] = U.rel_to_max(sdf.sdf(pts.cuda()).cpu(), want)
+    finally:
+        if saved is None:
+            os.environ.pop("AVC_FUSED_CHAIN", None)
+        else:
+            os.environ["AVC_FUSED_CHAIN"] = saved
+    return errs
+
+
+@pytest.mark.parametrize("name,P", [("tiny", 77), ("tiny", 5000), ("skiplast", 1000), ("shipped", 4099), ("b2", 20000),
+                                    ("tiny", P_PERSISTENT), ("skiplast", P_PERSISTENT), ("shipped", P_PERSISTENT),
+                                    ("b2", P_PERSISTENT), ("cfg1", P_PERSISTENT)])
 def test_fused_chain_sdf_query_matches_oracle(name, P):
     """engine 1 without a stash (sample placement, SDFNetwork.sdf) runs the whole value chain of a 128-point tile in ONE
     kernel (csrc/avc_chain.cu: activations resident in shared memory, sdf head folded into the last epilogue).  Covered:
-    widths 48 / 64 / 256, the skip concat inside the chain and at the head, ragged last tile, P < one tile."""
-    sdf_kw, col_kw, ren_kw, _ = U.CASES[name]
-    sconf, cconf, rconf = U.confs_from_kw(sdf_kw, col_kw, ren_kw)
-    sp, cp = U.synth_state(sdf_kw, col_kw, 5)
-    sdf, col, var, ren = U.build_product(sdf_kw, col_kw, ren_kw, sp, cp, 0.3, "cuda", engine=1)
-    pts = (torch.rand(P, 3, generator=torch.Generator().manual_seed(P)) - 0.5) * 2
-    got = sdf.sdf(pts.cuda()).cpu()
-    from oracle import neus
-    want = neus.sdf_value(sp, sconf, pts)
-    err = U.rel_to_max(got, want)
-    U.log_parity("fused_chain_sdf_query", {"case": name, "P": P, "rel_to_max": err})
-    assert err < 5e-5, err                     # two-term bf16 split operands (~16 mantissa bits); measured ~1e-5
+    widths 48 / 64 / 256, the skip concat inside the chain and at the head, ragged last tile, P < one tile, and at
+    P_PERSISTENT several tiles per CTA (the A tile is reloaded and the weight ring runs on across tiles) for chains of
+    4 and 9 layers, among them nets whose last chain layer has K <= 64 (tiny, skiplast, cfg1).  The layer-by-layer
+    tcgen05 launches (AVC_FUSED_CHAIN=0) are held to the same bar."""
+    errs = _chain_query_errors(name, P)
+    U.log_parity("fused_chain_sdf_query", {"case": name, "P": P, "tiles_per_cta": U.chain_tiles_per_cta(P),
+                                           "rel_to_max": errs["fused"], "rel_to_max_layered": errs["layered"]})
+    if P == P_PERSISTENT:
+        assert U.chain_tiles_per_cta(P) >= 5, U.chain_tiles_per_cta(P)
+    for variant, err in errs.items():
+        assert err < 5e-5, (variant, err)      # two-term bf16 split operands (~16 mantissa bits); measured ~1e-5
+
+
+def test_sdf_query_many_chunks():
+    """sdf_query splits P into chunks of max_rays_per_chunk * S points (avc_neus_sdf_query's p0 loop): 16 rays x 64
+    samples = 1024 points a chunk, 93 chunks with a ragged last one, each encoded and run through the chain."""
+    P = P_PERSISTENT
+    errs = _chain_query_errors("shipped", P, chunk=16)
+    U.log_parity("fused_chain_sdf_query", {"case": "shipped", "P": P, "chunk_points": 16 * 64,
+                                           "rel_to_max": errs["fused"], "rel_to_max_layered": errs["layered"]})
+    assert -(-P // (16 * 64)) >= 90
+    for variant, err in errs.items():
+        assert err < 5e-5, (variant, err)
 
 
 @pytest.mark.parametrize("name,bg,anneal", [("tiny", "ray", 1.0), ("skiplast", "none", 0.3), ("shipped", "ray", 1.0),

@@ -30,6 +30,25 @@ def log_parity(name: str, rec: dict):
         pass
 
 
+def sm_count() -> int:
+    return torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
+
+
+def nt_tiles_per_cta(M: int, N: int) -> int:
+    """Row tiles the first CTA of a tcgen05 NT launch walks (launch_gemm_tc_nt_bn's grid: min(tiles, SMs) persistent
+    CTAs, a whole number per column tile; BN = 64 for N <= 64, else 128)."""
+    BN = 64 if N <= 64 else 128
+    tiles_n, tiles_m = -(-N // BN), -(-M // 128)
+    m_stride = min(tiles_m * tiles_n, sm_count()) // tiles_n
+    return -(-tiles_m // m_stride)
+
+
+def chain_tiles_per_cta(P: int) -> int:
+    """128-point tiles the first CTA of the fused value chain walks (min(tiles, SMs) persistent CTAs)."""
+    tiles = -(-P // 128)
+    return -(-tiles // min(tiles, sm_count()))
+
+
 def flat_rel_l2(got: Dict[str, torch.Tensor], ref: Dict[str, torch.Tensor]) -> float:
     """rel-L2 error of the concatenated parameter gradient."""
     num = sum((got[k].double().cpu() - ref[k].double().cpu()).pow(2).sum().item() for k in ref)
@@ -42,7 +61,9 @@ def confs_from_kw(sdf_kw, col_kw, ren_kw):
     return sconf, neus.ColorConf(**col_kw), neus.RenderConf(**ren_kw)
 
 
-def build_product(sdf_kw, col_kw, ren_kw, sdf_state, col_state, variance, device, engine=0, chunk=4096):
+def build_product(sdf_kw, col_kw, ren_kw, sdf_state, col_state, variance, device, engine=0, chunk=4096,
+                  **renderer_kw):
+    """``renderer_kw``: further NeuSRenderer options (color_products, wgrad_products)."""
     import avatarclip_b200 as ab
     sdf = ab.SDFNetwork(**sdf_kw)
     col = ab.RenderingNetwork(**col_kw)
@@ -50,7 +71,7 @@ def build_product(sdf_kw, col_kw, ren_kw, sdf_state, col_state, variance, device
     sdf.load_state_dict(sdf_state)
     col.load_state_dict(col_state, strict=False)
     sdf, col, var = sdf.to(device), col.to(device), var.to(device)
-    ren = ab.NeuSRenderer(None, sdf, var, col, engine=engine, max_rays_per_chunk=chunk, **ren_kw)
+    ren = ab.NeuSRenderer(None, sdf, var, col, engine=engine, max_rays_per_chunk=chunk, **ren_kw, **renderer_kw)
     return sdf, col, var, ren
 
 
@@ -157,9 +178,10 @@ def synth_state(sdf_kw, col_kw, seed=0, tame=True):
     return sp, cp
 
 
-def run_case_gpu_vs_oracle(name: str, device="cuda", engine=0, seed=0, bg_kind="ray", anneal=1.0, chunk=4096,
-                           R: Optional[int] = None):
-    """Full comparison on a synthetic case.  Returns a report dict with worst errors and 'ok'."""
+def oracle_case(name: str, seed=0, bg_kind="ray", anneal=1.0, R: Optional[int] = None,
+                oracle_dtype=torch.float32) -> dict:
+    """Inputs of a synthetic case and the oracle's results on them: the full pipeline (sample placement) in fp32, as
+    the reference runs it, then the fine pass and its backward on the oracle's own depths in ``oracle_dtype``."""
     sdf_kw, col_kw, ren_kw, Rdef = CASES[name]
     R = R or Rdef
     sconf, cconf, rconf = confs_from_kw(sdf_kw, col_kw, ren_kw)
@@ -168,32 +190,50 @@ def run_case_gpu_vs_oracle(name: str, device="cuda", engine=0, seed=0, bg_kind="
     o, d, near, far, jit = make_rays(R, seed + 1)
     g = torch.Generator().manual_seed(seed + 2)
     bg = {"none": None, "white": torch.ones(1, 3), "ray": torch.rand(R, 1, generator=g)}[bg_kind]
-    sdf, col, var, ren = build_product(sdf_kw, col_kw, ren_kw, sp, cp, variance, device, engine=engine, chunk=chunk)
+    rays = (o, d, near, far, jit, bg, anneal)
+    oout, _ = oracle_run(sconf, cconf, rconf, sp, cp, variance, *rays)
+    z = oout["z_vals"].detach()
+    cot = cotangents(oout)
+    oout2, ograds = oracle_run(sconf, cconf, rconf, sp, cp, variance, *rays, cot=cot, z_vals=z, dtype=oracle_dtype)
+    return {"name": name, "R": R, "sp": sp, "cp": cp, "variance": variance, "rays": rays, "placement": oout, "z": z,
+            "cot": cot, "fine": oout2, "grads": ograds, "oracle_dtype": str(oracle_dtype).replace("torch.", "")}
+
+
+def run_case_gpu_vs_oracle(name: str, device="cuda", engine=0, seed=0, bg_kind="ray", anneal=1.0, chunk=4096,
+                           R: Optional[int] = None, oracle_dtype=torch.float32, oracle: Optional[dict] = None,
+                           **renderer_kw):
+    """Full comparison on a synthetic case.  Returns a report dict with worst errors and 'ok'.  ``oracle``: the result
+    of oracle_case for the same case (computed here when None; the other case arguments are then ignored).
+    ``renderer_kw``: further NeuSRenderer options."""
+    if oracle is None:
+        oracle = oracle_case(name, seed, bg_kind, anneal, R, oracle_dtype)
+    sdf_kw, col_kw, ren_kw, _ = CASES[oracle["name"]]
+    R = oracle["R"]
+    sp, cp, variance, rays = oracle["sp"], oracle["cp"], oracle["variance"], oracle["rays"]
+    sdf, col, var, ren = build_product(sdf_kw, col_kw, ren_kw, sp, cp, variance, device, engine=engine, chunk=chunk,
+                                       **renderer_kw)
 
     # (1) placement
-    pout, _ = product_run(ren, sdf, col, var, o, d, near, far, jit, bg, anneal, device=device)
-    oout, _ = oracle_run(sconf, cconf, rconf, sp, cp, variance, o, d, near, far, jit, bg, anneal)
+    pout, _ = product_run(ren, sdf, col, var, *rays, device=device)
+    oout = oracle["placement"]
     dz = (pout["z_vals"] - oout["z_vals"].detach()).abs().max(dim=1)[0]
     # fp32 round-off in the coarse SDF moves inverse-CDF samples by up to ~1e-3 even between the oracle's own
     # fp32 and fp64 runs (measured: DESIGN.md 'parity definition'); flips show up as much larger jumps.
-    rep = {"case": name, "R": R, "placement_frac_3e-3": (dz < 3e-3).float().mean().item(),
+    rep = {"case": oracle["name"], "R": R, "placement_frac_3e-3": (dz < 3e-3).float().mean().item(),
            "placement_median_dz": dz.median().item(), "placement_max_dz": dz.max().item()}
     dc = (pout["extra_color_fine"] - oout["extra_color_fine"].detach()).abs().max(dim=1)[0]
     rep["full_render_frac_rays_1e-3"] = (dc < 1e-3).float().mean().item()
 
     # (2) fine pass + backward on the oracle's depths
-    z = oout["z_vals"].detach()
-    cot = cotangents(oout)
-    oout2, ograds = oracle_run(sconf, cconf, rconf, sp, cp, variance, o, d, near, far, jit, bg, anneal, cot=cot,
-                               z_vals=z)
-    pout2, pgrads = product_run(ren, sdf, col, var, o, d, near, far, jit, bg, anneal, cot=cot, z_vals=z,
-                                device=device)
+    oout2, ograds = oracle["fine"], oracle["grads"]
+    pout2, pgrads = product_run(ren, sdf, col, var, *rays, cot=oracle["cot"], z_vals=oracle["z"], device=device)
     rep["out_err"] = {k: rel_to_max(pout2[k], oout2[k]) for k in COT_KEYS + ["mid_z_vals", "inside_sphere"]}
     rep["grad_err"] = {k: rel_to_max(pgrads[k], ograds[k]) for k in ograds}
     rep["worst_out"] = max(rep["out_err"].values())
     rep["worst_grad"] = max(rep["grad_err"].values())
     rep["grad_rel_l2"] = flat_rel_l2(pgrads, ograds)
     rep["engine"] = engine
+    rep["oracle_dtype"] = oracle["oracle_dtype"]
     # bars (north_star: 1e-3 relative on the rendered outputs; gradients: VERDICT r1 asks <= 1e-3 rel-L2):
     #   fine pass on identical depths: every output within OUT_BAR (rel-to-max), flat gradient within 1e-3 rel-L2;
     #   full pipeline (own placement): >= 99 % of rays within 1e-3 in colour, >= 97 % within 3e-3 in depth -- the
@@ -201,7 +241,7 @@ def run_case_gpu_vs_oracle(name: str, device="cuda", engine=0, seed=0, bg_kind="
     out_bar = 1e-4 if engine == 0 else 1e-3
     rep["ok"] = (rep["worst_out"] < out_bar and rep["grad_rel_l2"] < 1e-3 and rep["placement_frac_3e-3"] >= 0.97
                  and rep["full_render_frac_rays_1e-3"] >= 0.99)
-    log_parity("run_case", {k: rep[k] for k in ("case", "engine", "R", "worst_out", "worst_grad", "grad_rel_l2",
-                                                "placement_frac_3e-3", "placement_max_dz",
+    log_parity("run_case", {k: rep[k] for k in ("case", "engine", "R", "oracle_dtype", "worst_out", "worst_grad",
+                                                "grad_rel_l2", "placement_frac_3e-3", "placement_max_dz",
                                                 "full_render_frac_rays_1e-3")})
     return rep
